@@ -28,6 +28,11 @@ falls back to the port alone and says so (`reference_kind`).
   --graph T          time CUDA-graph replays of T captured steps (SwarmEngine.capture_steps) instead of a Python
                      loop over step(): what the launch-bound batch sizes BASELINE names (4096 x 8 drones) need
   named_sizes        the default run also reports C2 / C3 / C4-shard / C5 at BASELINE's own env counts
+  --dump-outputs DIR after the timed steps, write what their last step handed its caller (every output field of
+                     the step: obs, reward, dist, the flag arrays, __all__ flags, global_state) as DIR/<name>.npy
+                     (float32; float64 stays float64) for a seeded sample of env instances (DIR/env_index.npy) that
+                     keeps the dump under 64 MB.  Inputs are fixed by the arguments, so two builds run with the
+                     same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -205,6 +210,28 @@ def run_reference_arm(args, kind, cfg, wl_name, default_envs):
     print(json.dumps(line), flush=True)
 
 
+DUMP_BYTES = 48 << 20   # --dump-outputs budget (files + headers stay under 64 MB)
+
+
+def dump_outputs(eng, out_dir):
+    """The step's output fields (_abi.HOST_OUT_FIELDS present on this engine) of a fixed sample of env instances,
+    as out_dir/<name>.npy; the sampled env indices as out_dir/env_index.npy."""
+    import torch
+    from swarm_b200 import _abi
+
+    fields = {n: getattr(eng, n) for n in _abi.HOST_OUT_FIELDS if getattr(eng, n, None) is not None}
+    per_env = 8 + sum(t[0].numel() * (8 if t.dtype == torch.float64 else 4) for t in fields.values())
+    n = min(eng.E, DUMP_BYTES // per_env)
+    idx = np.arange(eng.E) if n == eng.E else np.sort(np.random.default_rng(0).choice(eng.E, n, replace=False))
+    sel = torch.from_numpy(idx).to(eng.device)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "env_index.npy"), idx.astype(np.float64))
+    for name, t in fields.items():
+        t = t.index_select(0, sel)
+        t = t if t.dtype == torch.float64 else t.to(torch.float32)
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy())
+
+
 def kernel_name(kind, n, envs):
     """The kernel `swarm_step` selects for this shape (swarm_abi.cu: rot_eligible / rotx_eligible / launch)."""
     if kind == "swarm" and n in (8, 16, 32):
@@ -250,7 +277,16 @@ def main():
     ap.add_argument("--graph", type=int, default=0, metavar="T",
                     help="time CUDA-graph replays of T captured steps instead of a Python loop over step()")
     ap.add_argument("--no-named-sizes", action="store_true", help="skip the block at BASELINE's own env counts")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (rank 0's env instances, a seeded "
+                         "sample of them where all would exceed 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.graph and args.steps % args.graph:
+        ap.error("--steps must be a multiple of --graph (each replay runs --graph steps)")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours (the reference arm has no device outputs)")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     kind, cfg, default_envs = WORKLOADS[args.workload]
@@ -300,7 +336,8 @@ def main():
 
     def timed(e, steps, warmup, sample_clocks, graph_T=None, acts=None):
         """W untimed + K timed steps, CUDA events on the launching stream, max over ranks.  graph_T > 0: the K steps
-        are K / T replays of a CUDA graph of T captured steps (K rounded down to a multiple of T)."""
+        are K / T replays of a CUDA graph of T captured steps.  main() only passes a --steps that is a multiple of
+        --graph; the secondary legs (pre-warm, DR off, named sizes) have K rounded down to a multiple of T (at least T)."""
         graph_T = args.graph if graph_T is None else graph_T
         acts = actions if acts is None else acts
         E_, N_ = e.E, e.N
@@ -355,6 +392,8 @@ def main():
         timed(eng, args.steps, args.warmup, True)
     steps_done = int(steps_done)
     value = agent_steps_all / (elapsed_ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(eng, args.dump_outputs)   # before the host-buffer arm steps the same engine again
 
     dr_off = None
     if dr_enabled(args) and not args.no_dr_off:
