@@ -99,7 +99,7 @@ def test_dump_outputs_are_the_oracle_step_after_the_last_timed_step(tmp_path):
     another step, or rows paired with the wrong env_index entries, differs."""
     import torch
     import swarm_oracle as so
-    from parity_util import assert_biteq, bits, obs_row_ok_up_to_ties
+    from parity_util import assert_biteq
 
     E, N, W, K = 16384, 32, 3, 7
     cfg = {"num_drones": N, "num_obstacles": 8}
@@ -124,6 +124,4 @@ def test_dump_outputs_are_the_oracle_step_after_the_last_timed_step(tmp_path):
         assert_biteq(name, a, getattr(o, name), K)
     valid = o.obs_valid.astype(bool)
     assert valid.any()
-    for e, i in np.argwhere((bits(obs) != bits(o.obs)).any(axis=2) & valid):   # exact distance ties may order differently
-        assert obs_row_ok_up_to_ties("swarm", {**so.DEFAULTS, **cfg}, o.positions[e], o.velocities[e], o.goal[e],
-                                     o.obstacles[e], i, obs[e, i]), (e, i)
+    assert_biteq("obs", obs[valid], o.obs[valid], K)

@@ -4,8 +4,9 @@ fixtures recorded from the unmodified reference and (b) the C oracle on seeded i
 Bar (BASELINE.json north_star): fp32 state / obs / reward within 1e-5 relative over 1000
 steps, flags bit-exact up to counted 1-ulp threshold cases.  What is asserted here is
 stronger: state, observations, float64 rewards, distances, flags, global_state and the reset
-draws are BIT-EXACT; the only tolerated difference is the order of exactly tied distances in
-the k-nearest blocks (np.argsort is not stable, SURVEY T5), which is validated and counted.
+draws are BIT-EXACT.  Against the golden fixtures the order of exactly tied distances in the
+k-nearest blocks is validated instead (np.argsort is not stable, SURVEY T5); against the C oracle
+it is not: the oracle and the kernels both put the lowest index first on a tie.
 """
 import numpy as np
 import pytest
@@ -130,7 +131,7 @@ def test_parked_drones_masked_rotation_pass(N, world, dr):
     states: random subsets parked, parked drones sitting inside an active drone's collision sphere, and an active
     drone whose three nearest are all parked-and-touching with / without an active one just behind them."""
     import swarm_oracle as so
-    from parity_util import assert_biteq, obs_row_ok_up_to_ties
+    from parity_util import assert_biteq
 
     cfg = {"num_drones": N, "num_obstacles": 8, "world_size": world, "max_steps": 50}
     E, T = 96, 10
@@ -165,7 +166,6 @@ def test_parked_drones_masked_rotation_pass(N, world, dr):
     o.active[:] = active
     o.observe()
     b.eng.set_state(pos, o.velocities, o.goal, o.obstacles, alive=active)
-    ties = 0
     for t in range(-1, T):
         if t >= 0:
             act = rng.uniform(-0.3, 0.3, size=(E, N, 3)).astype(np.float32)
@@ -176,23 +176,18 @@ def test_parked_drones_masked_rotation_pass(N, world, dr):
                                                     "all_terminated", "all_truncated")):
             assert_biteq(name, getattr(b, name), getattr(o, name), t)
         valid = o.obs_valid.astype(bool)
-        bo, oo = b.obs, o.obs
-        for e, i in np.argwhere((pu.bits(bo) != pu.bits(oo)).any(axis=2) & valid):
-            assert not dr, f"obs row differs under randomisation at step {t} env {e} drone {i}"
-            assert obs_row_ok_up_to_ties("swarm", {**so.DEFAULTS, **cfg}, o.positions[e], o.velocities[e], o.goal[e],
-                                         o.obstacles[e], i, bo[e, i]), f"obs row beyond ties at step {t} env {e} drone {i}"
-            ties += 1
+        assert_biteq("obs", b.obs[valid], o.obs[valid], t)
         if t == 0:   # the injected layouts did what they were built for
             assert len(behind) >= 3 and len(touching) >= 3
             assert (o.collision[behind, 0] == 1).all()       # the active 4th-nearest behind three parked ones counts
             assert (o.collision[touching, 0] == 0).sum() >= 3  # parked neighbours alone never collide
-    assert int(o.active.sum()) < E * N and ties < 10
+    assert int(o.active.sum()) < E * N
 
 
 @pytest.mark.parametrize("kind,cfg,E,T,scale", CASES)
 def test_cuda_matches_oracle_seeded(kind, cfg, E, T, scale):
     import swarm_oracle as so
-    from parity_util import assert_biteq, obs_row_ok_up_to_ties
+    from parity_util import assert_biteq
 
     b = _backend(E, cfg, kind=kind)
     o = so.OracleSwarm(E, cfg, kind=kind)
@@ -203,7 +198,6 @@ def test_cuda_matches_oracle_seeded(kind, cfg, E, T, scale):
     o.reset()
     rng = np.random.default_rng(42)
     N = o.N
-    ties = 0
     for t in range(-1, T):
         if t >= 0:
             if t % 3 == 2:  # goal seeking: parks drones, reaches goals
@@ -219,13 +213,8 @@ def test_cuda_matches_oracle_seeded(kind, cfg, E, T, scale):
                      "global_state", "active"):
             assert_biteq(name, getattr(b, name), getattr(o, name), t)
         valid = o.obs_valid.astype(bool)
-        bo, oo = b.obs, o.obs
-        diff = np.argwhere((pu.bits(bo) != pu.bits(oo)).any(axis=2) & valid)
-        for e, i in diff:
-            assert obs_row_ok_up_to_ties(kind, {**so.DEFAULTS, **cfg}, o.positions[e], o.velocities[e], o.goal[e],
-                                         o.obstacles[e], i, bo[e, i]), f"obs row beyond ties at step {t} env {e} drone {i}"
-            ties += 1
-    print(f"{kind} {cfg}: E={E} T={T} bit-exact; tie rows {ties}")
+        assert_biteq("obs", b.obs[valid], o.obs[valid], t)
+    print(f"{kind} {cfg}: E={E} T={T} bit-exact")
 
 
 def test_no_auto_reset_and_dead_env_contract():
@@ -770,7 +759,7 @@ LONG_HORIZON = [
 @pytest.mark.parametrize("name,cfg,E,T", LONG_HORIZON)
 def test_cuda_matches_oracle_over_1000_steps(name, cfg, E, T):
     """1000 consecutive steps (auto-reset on, U(-1, 1) actions) of 256 env instances per BASELINE shape: every
-    array bit for bit at every step; obs rows that differ are validated as exact-distance ties and counted."""
+    array bit for bit at every step, the obs rows of the valid agents included."""
     import os
     import swarm_oracle as so
     from parity_util import assert_biteq
@@ -784,7 +773,6 @@ def test_cuda_matches_oracle_over_1000_steps(name, cfg, E, T):
     rng = np.random.default_rng(321)
     N = o.N
     threads = len(os.sched_getaffinity(0))
-    ties = 0
     fields = ("positions", "velocities", "goal", "obstacles", "step_count", "reward", "dist", "terminated", "truncated",
               "reached", "collision", "obs_valid", "all_terminated", "all_truncated", "global_state", "active")
     for t in range(-1, T):
@@ -795,14 +783,10 @@ def test_cuda_matches_oracle_over_1000_steps(name, cfg, E, T):
         for fname in fields:
             assert_biteq(fname, getattr(b, fname), getattr(o, fname), t)
         valid = o.obs_valid.astype(bool)
-        bo, oo = b.obs, o.obs
-        for e, i in np.argwhere((pu.bits(bo) != pu.bits(oo)).any(axis=2) & valid):
-            assert pu.obs_row_ok_up_to_ties("swarm", {**so.DEFAULTS, **cfg}, o.positions[e], o.velocities[e], o.goal[e],
-                                            o.obstacles[e], i, bo[e, i]), f"obs row beyond ties at step {t} env {e} drone {i}"
-            ties += 1
+        assert_biteq("obs", b.obs[valid], o.obs[valid], t)
     st = b.eng.stats()
     assert st["env_steps"] == E * T
-    print(f"{name}: {E} envs x {N} drones x {T} steps bit-exact; episodes {st['episodes']}, tie rows {ties}")
+    print(f"{name}: {E} envs x {N} drones x {T} steps bit-exact; episodes {st['episodes']}")
 
 
 @pytest.mark.parametrize("name,cfg,E,T,dr", FULL_SIZE)
@@ -827,7 +811,6 @@ def test_cuda_matches_oracle_at_full_baseline_size(name, cfg, E, T, dr):
     rng = np.random.default_rng(123)
     N = o.N
     threads = len(os.sched_getaffinity(0))
-    ties = 0
     for t in range(-1, T):
         if t >= 0:
             act = rng.uniform(-1.0, 1.0, size=(E, N, 3)).astype(np.float32)
@@ -838,13 +821,7 @@ def test_cuda_matches_oracle_at_full_baseline_size(name, cfg, E, T, dr):
                       "global_state", "active"):
             assert_biteq(fname, getattr(b, fname), getattr(o, fname), t)
         valid = o.obs_valid.astype(bool)
-        bo, oo = b.obs, o.obs
-        diff = np.argwhere((pu.bits(bo) != pu.bits(oo)).any(axis=2) & valid)
-        for e, i in diff:
-            assert dr_cfg is None, "with sensor noise a tie-ordered row cannot be re-derived from the state"
-            assert pu.obs_row_ok_up_to_ties("swarm", {**so.DEFAULTS, **cfg}, o.positions[e], o.velocities[e], o.goal[e],
-                                            o.obstacles[e], i, bo[e, i]), f"obs row beyond ties at step {t} env {e} drone {i}"
-            ties += 1
+        assert_biteq("obs", b.obs[valid], o.obs[valid], t)
     st = b.eng.stats()
     assert st["env_steps"] == E * T
-    print(f"{name}: {E} envs x {N} drones x {T} steps bit-exact; episodes {st['episodes']}, tie rows {ties}")
+    print(f"{name}: {E} envs x {N} drones x {T} steps bit-exact; episodes {st['episodes']}")
