@@ -64,7 +64,7 @@ __device__ __forceinline__ void pair_block8(const float4* __restrict__ tpos, int
     }
 #pragma unroll
     for (int u = 0; u < 8; ++u) {
-        topk_insert<KT>(valid[u] ? d[u] : F32_INF, jb + u, nd, nj);
+        topk_insert<KT>(valid[u] ? d[u] : TOPK_EMPTY, jb + u, nd, nj);
         if (FORM != 0) {
             const double err = fabs(__dsub_rn((double)d[u], d_star));
             if (FORM == 1) r[u] = __dadd_rn(r[u], err);
@@ -95,7 +95,7 @@ __device__ __forceinline__ void obst_block4(const float4* __restrict__ tobs, int
         for (int u = 0; u < 4; ++u) d[u] = __fsqrt_rn(s[u]);
     }
 #pragma unroll
-    for (int u = 0; u < 4; ++u) topk_insert<ST>(valid[u] ? d[u] : F32_INF, mb + u, od, om);
+    for (int u = 0; u < 4; ++u) topk_insert<ST>(valid[u] ? d[u] : TOPK_EMPTY, mb + u, od, om);
 }
 
 // KT / ST: capacity of the k-nearest lists (>= K, S).  nj holds "other" indices jp (see above).
@@ -106,9 +106,9 @@ __device__ __forceinline__ void scan_drone(const DevParams& P, const float4* __r
                                            float (&od)[ST], int (&om)[ST], ScanOut& out) {
     const int N = P.N, M = P.M;
 #pragma unroll
-    for (int q = 0; q < KT; ++q) { nd[q] = F32_INF; nj[q] = -1; }
+    for (int q = 0; q < KT; ++q) { nd[q] = TOPK_EMPTY; nj[q] = -1; }
 #pragma unroll
-    for (int q = 0; q < ST; ++q) { od[q] = F32_INF; om[q] = -1; }
+    for (int q = 0; q < ST; ++q) { od[q] = TOPK_EMPTY; om[q] = -1; }
     out.pair_hit = false;
     out.form_sum = 0.0;
     out.form_n = 0;
@@ -119,7 +119,7 @@ __device__ __forceinline__ void scan_drone(const DevParams& P, const float4* __r
         for (; mb + 4 <= M; mb += 4) obst_block4<ST, true>(tobs, mb, M, px, py, pz, od, om);
         if (mb < M) obst_block4<ST, false>(tobs, mb, M, px, py, pz, od, om);
     }
-    out.obst_hit = od[0] <= P.thr_obst;  // nearest obstacle decides; +inf when M == 0
+    out.obst_hit = od[0] <= P.thr_obst;  // nearest obstacle decides; TOPK_EMPTY (a NaN) when M == 0
     if (KIND == SWARM_KIND_SINGLE) return;
 
     // ---- drones: _nearest_neighbor_features (:245-271) over ALL j != i; pair part of
@@ -1343,11 +1343,11 @@ __global__ void __launch_bounds__(kThreadsPerCta, kMinBlocksPerSm) swarm_env_ker
                     (w ? par_w : par_nw)[r0 * srow] = dd;
                 }
             }
-            // pad the row to a multiple of 8 columns with +inf so B2 runs whole blocks only
+            // pad the row to a multiple of 8 columns with non-candidates so B2 runs whole blocks only
             if (lane_ok) {
 #pragma unroll
                 for (int u = 0; u < 7; ++u)
-                    if (n_others + u < n_pad) drow[n_others + u] = F32_INF;
+                    if (n_others + u < n_pad) drow[n_others + u] = TOPK_EMPTY;
             }
         }
         __syncwarp();
@@ -1355,7 +1355,7 @@ __global__ void __launch_bounds__(kThreadsPerCta, kMinBlocksPerSm) swarm_env_ker
         // ================ B2: own row in ascending order: k-nearest (+ formation) ================
         float nd[KT]; int nj[KT];
 #pragma unroll
-        for (int q = 0; q < KT; ++q) { nd[q] = F32_INF; nj[q] = -1; }
+        for (int q = 0; q < KT; ++q) { nd[q] = TOPK_EMPTY; nj[q] = -1; }
         bool pair_hit = false;
         double form_sum = 0.0;
         int form_n = 0;
@@ -1384,7 +1384,7 @@ __global__ void __launch_bounds__(kThreadsPerCta, kMinBlocksPerSm) swarm_env_ker
                     }
 #pragma unroll
                     for (int u = 0; u < 8; ++u) {
-                        const float d = drow[cb + u];  // +inf in the padding columns: never selected
+                        const float d = drow[cb + u];  // TOPK_EMPTY in the padding columns: never selected
                         topk_insert<KT>(d, cb + u, nd, nj);
                         r8[u] = __dadd_rn(r8[u], fabs(__dsub_rn((double)d, d_star)));
                     }
@@ -1437,7 +1437,7 @@ __global__ void __launch_bounds__(kThreadsPerCta, kMinBlocksPerSm) swarm_env_ker
         // ---- obstacles: _nearest_obstacle_features (:273-291) + obstacle part of _collision_mask
         float od[ST]; int om[ST];
 #pragma unroll
-        for (int q = 0; q < ST; ++q) { od[q] = F32_INF; om[q] = -1; }
+        for (int q = 0; q < ST; ++q) { od[q] = TOPK_EMPTY; om[q] = -1; }
         {
             int mb = 0;
 #pragma unroll 1

@@ -774,7 +774,7 @@ __global__ void __launch_bounds__(rot_warps(NT, DRM != 0) * 32, rot_min_blocks(N
                 }
                 if (__any_sync(FULL_MASK, mine && (k2 ^ k3) <= IDX)) {
 #pragma unroll
-                    for (int q = 0; q < 3; ++q) { nd[q] = F32_INF; nj[q] = 0; }
+                    for (int q = 0; q < 3; ++q) { nd[q] = TOPK_EMPTY; nj[q] = 0; }
                     const float4* te = tab2 + 2 * e_base;
 #pragma unroll 1
                     for (int j = 0; j < N; ++j) {
@@ -890,7 +890,7 @@ __global__ void __launch_bounds__(rot_warps(NT, DRM != 0) * 32, rot_min_blocks(N
 #endif
                 if (__any_sync(FULL_MASK, mine && bad_o)) {  // an undecided obstacle order: the reference's loop as written
 #pragma unroll
-                    for (int q = 0; q < 4; ++q) { od[q] = F32_INF; om[q] = 0; }
+                    for (int q = 0; q < 4; ++q) { od[q] = TOPK_EMPTY; om[q] = 0; }
 #pragma unroll 1
                     for (int m = 0; m < M; ++m) {
                         const float4 o = tobs[m];
@@ -904,7 +904,7 @@ __global__ void __launch_bounds__(rot_warps(NT, DRM != 0) * 32, rot_min_blocks(N
                 // the reference's loops as written: ascending j, strict '<' (lowest index wins ties),
                 // collision / formation over ACTIVE pairs only, np.mean's pairwise summation order
 #pragma unroll
-                for (int q = 0; q < 3; ++q) { nd[q] = F32_INF; nj[q] = 0; }
+                for (int q = 0; q < 3; ++q) { nd[q] = TOPK_EMPTY; nj[q] = 0; }
                 pair_hit = false;
                 const unsigned em = (alive_mask & env_lanes) >> e_base;  // bit j: drone j of this env active
                 const int n_f = alive ? n_alive_env - 1 : 0;
@@ -941,7 +941,7 @@ __global__ void __launch_bounds__(rot_warps(NT, DRM != 0) * 32, rot_min_blocks(N
                 form_sum = res;
                 form_n = n_f;
 #pragma unroll
-                for (int q = 0; q < 4; ++q) { od[q] = F32_INF; om[q] = 0; }
+                for (int q = 0; q < 4; ++q) { od[q] = TOPK_EMPTY; om[q] = 0; }
 #pragma unroll 1
                 for (int m = 0; m < M; ++m) {
                     const float4 o = tobs[m];

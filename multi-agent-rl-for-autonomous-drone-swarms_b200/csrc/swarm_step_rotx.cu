@@ -186,7 +186,7 @@ swarm_step_rotx_kernel(const DevParams P) {
                 ctrl_delay = (int)d1.w;
             }
             const float* act = reinterpret_cast<const float*>(in_pos + 2 * N);
-            bool nan_any = false;
+            unsigned nan_n = 0u;
 #pragma unroll
             for (int s = 0; s < NS; ++s) {
                 const float4 p = SWARM_ROTX_DIRECT ? lp[s] : in_pos[s * 32 + lane];
@@ -216,7 +216,7 @@ swarm_step_rotx_kernel(const DevParams P) {
                         wp[0] = sx; wp[1] = sy; wp[2] = sz;
                     }
                     ax = clipf(ax, -1.0f, 1.0f); ay = clipf(ay, -1.0f, 1.0f); az = clipf(az, -1.0f, 1.0f);
-                    nan_any = nan_any || !(ax == ax && ay == ay && az == az);   // (np.clip lets NaN through; counted)
+                    nan_n += (ax == ax && ay == ay && az == az) ? 0u : 1u;   // (np.clip lets NaN through; counted)
                     if (DR) {  // thrust noise: a <- a * (1 + sigma z), one normal per axis
                         const uint4 r = philox4x32_7(genv, ekey, (unsigned)sc, (unsigned)(s * 32 + lane) | (DR_STREAM_A << 16), P);
                         ax = __fmul_rn(ax, __fmaf_rn(P.dr_std_thrust, dr_normal(P.dr_qtable, dr_field(r, 0)), 1.0f));
@@ -241,9 +241,11 @@ swarm_step_rotx_kernel(const DevParams P) {
                 pz[s] = clipf(pz[s], -c_bound, c_bound);
                 vx[s] = v.x; vy[s] = v.y; vz[s] = v.z;
             }
-            {   // NaN-action guard counter (rare: the vote is all a clean step pays); per lane: drones, not components
-                const unsigned nan_m = __ballot_sync(FULL_MASK, nan_any);
-                if (nan_m != 0u && lane == 0) wstats[SWARM_STAT_NAN_ACTIONS] += (unsigned long long)__popc(nan_m);
+            // NaN-action guard counter (rare: the vote is all a clean step pays): drones, not components -- a lane
+            // holds NS drones, so the lanes' counts are summed
+            if (__any_sync(FULL_MASK, nan_n != 0u)) {
+                const unsigned n = __reduce_add_sync(FULL_MASK, nan_n);
+                if (lane == 0) wstats[SWARM_STAT_NAN_ACTIONS] += (unsigned long long)n;
             }
         } else {
             // ================================ reset (:65-80) ================================
@@ -486,8 +488,11 @@ swarm_step_rotx_kernel(const DevParams P) {
             for (int s = 0; s < NS; ++s)
                 // (keys sharing a bucket are settled per drone in the tail: among keys 0-2 only the ORDER is open,
                 //  a 3rd/4th-key collision triggers an exact neighbour rescan of that slot pass; only a distance
-                //  below 2^-14 -- fast sqrt / exact-sum preconditions -- sends the whole item to the exact path)
-                bad = bad || (STEP && (!(acc[s] == acc[s]) || k0[s] < 0x38800000u));
+                //  below 2^-14 -- fast sqrt / exact-sum preconditions -- or a NaN position sends the whole item to the
+                //  exact path.  The integer float32 -> float64 conversions of the rounds turn NaN into a finite value,
+                //  so a NaN drone does not show up as a NaN formation sum here: its position is checked instead)
+                bad = bad || (STEP && (!(acc[s] == acc[s]) || k0[s] < 0x38800000u ||
+                                       !(px[s] == px[s] && py[s] == py[s] && pz[s] == pz[s])));
         };
         if (all_alive) rotation_pass(std::false_type{});
         else rotation_pass(std::true_type{});
@@ -542,7 +547,7 @@ swarm_step_rotx_kernel(const DevParams P) {
                     // Redo the neighbour selection of this slot pass exactly (ascending j, strict '<'); the
                     // formation sum is exact regardless.
 #pragma unroll
-                    for (int q = 0; q < 3; ++q) { nd[q] = F32_INF; nj[q] = 0; }
+                    for (int q = 0; q < 3; ++q) { nd[q] = TOPK_EMPTY; nj[q] = 0; }
 #pragma unroll 1
                     for (int j = 0; j < N; ++j) {
                         if (j == me) continue;
@@ -586,7 +591,7 @@ swarm_step_rotx_kernel(const DevParams P) {
                 // exact path: the reference's loops as written (ascending j, strict '<', active pairs, numpy's
                 // pairwise summation order)
 #pragma unroll
-                for (int q = 0; q < 3; ++q) { nd[q] = F32_INF; nj[q] = 0; }
+                for (int q = 0; q < 3; ++q) { nd[q] = TOPK_EMPTY; nj[q] = 0; }
                 const int n_f = alive[0] ? n_alive_env - 1 : 0;
                 const int nf8 = n_f >= 8 ? (n_f & ~7) : 0;
                 double r8[8];
@@ -664,7 +669,7 @@ swarm_step_rotx_kernel(const DevParams P) {
             }
             if (__any_sync(FULL_MASK, bad_o)) {
 #pragma unroll
-                for (int q = 0; q < 4; ++q) { od[q] = F32_INF; om[q] = 0; }
+                for (int q = 0; q < 4; ++q) { od[q] = TOPK_EMPTY; om[q] = 0; }
 #pragma unroll 1
                 for (int m = 0; m < M; ++m) {
                     const float4 o = tobs[m];

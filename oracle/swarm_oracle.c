@@ -342,6 +342,13 @@ static int obs_dim(const OracleConfig *c) {
 /* Observation pieces                                                         */
 /* ------------------------------------------------------------------------- */
 
+/* np.argsort's order of two distances: a ranks strictly after b.  NaN sorts after every number (+inf
+ * included), so a NaN candidate is picked only when there are not enough numbers; NaNs tie with each other. */
+static int ranks_after(float a, float b) {
+    if (isnan(a)) return !isnan(b);
+    return a > b;
+}
+
 /* _nearest_obstacle_features  drone_swarm_env.py:273-291 / single_drone_env.py:142-159 */
 static void nearest_obstacle_features(const OracleConfig *c, const float *own, const float *obst,
                                       float *out) {
@@ -355,10 +362,10 @@ static void nearest_obstacle_features(const OracleConfig *c, const float *own, c
         dist[m] = norm_axis(rx, ry, rz);
         order[m] = m;
     }
-    /* stable insertion sort == argsort with lowest-index tie break */
+    /* stable insertion sort == argsort with lowest-index tie break, NaN last */
     for (int a = 1; a < M; ++a) {
         int key = order[a], b = a - 1;
-        while (b >= 0 && dist[order[b]] > dist[key]) { order[b + 1] = order[b]; --b; }
+        while (b >= 0 && ranks_after(dist[order[b]], dist[key])) { order[b + 1] = order[b]; --b; }
         order[b + 1] = key;
     }
     int k = S < M ? S : M;
@@ -391,7 +398,7 @@ static void nearest_neighbor_features(const OracleConfig *c, const float *pos, i
     }
     for (int a = 1; a < n; ++a) {
         int key = order[a], b = a - 1;
-        while (b >= 0 && dist[order[b]] > dist[key]) { order[b + 1] = order[b]; --b; }
+        while (b >= 0 && ranks_after(dist[order[b]], dist[key])) { order[b + 1] = order[b]; --b; }
         order[b + 1] = key;
     }
     int k = K < n ? K : n;
