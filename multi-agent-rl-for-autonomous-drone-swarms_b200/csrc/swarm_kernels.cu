@@ -359,68 +359,15 @@ __global__ void __launch_bounds__(kThreadsPerCta, kMinBlocksPerSm) swarm_env_ker
                     if (alive) {
                         float ax = P.actions[a * 3 + 0], ay = P.actions[a * 3 + 1], az = P.actions[a * 3 + 2];
                         const bool clip_cmd = !PHYS;   // (the physics env neither clips nor casts the action, :336)
-                        if (DR && P.dr_delay_hist > 0) {
-                            // control delay: apply the command submitted ctrl_delay steps ago (zero while the episode
-                            // is younger), then file the one submitted now in ring slot step_count % H
-                            const int H = P.dr_delay_hist;
-                            float* ring = P.act_hist + (long long)env * H * N * 3 + i * 3;
-                            const float sx = ax, sy = ay, sz = az;
-                            if (ctrl_delay > 0) {
-                                if (sc < ctrl_delay) {
-                                    ax = 0.f; ay = 0.f; az = 0.f;
-                                } else {
-                                    const float* hp = ring + (long long)((sc - ctrl_delay) % H) * N * 3;
-                                    ax = hp[0]; ay = hp[1]; az = hp[2];
-                                }
-                            }
-                            float* wp = ring + (long long)(sc % H) * N * 3;
-                            wp[0] = sx; wp[1] = sy; wp[2] = sz;
-                        }
+                        if (DR && P.dr_delay_hist > 0) delayed_command(P, env, N, i, sc, ctrl_delay, ax, ay, az);
                         if (clip_cmd) { ax = clipf(ax, -1.0f, 1.0f); ay = clipf(ay, -1.0f, 1.0f); az = clipf(az, -1.0f, 1.0f); }
                         if (!(ax == ax && ay == ay && az == az)) ++st_nan;   // NaN-action guard counter
-                        if (DR) {  // thrust noise: a <- a * (1 + sigma z), one normal per axis
+                        if (DR) {
                             const uint4 r = philox4x32_7(genv, ekey, (unsigned)sc, (unsigned)i | (DR_STREAM_A << 16), P);
-                            ax = __fmul_rn(ax, __fmaf_rn(P.dr_std_thrust, dr_normal(P.dr_qtable, dr_field(r, 0)), 1.0f));
-                            ay = __fmul_rn(ay, __fmaf_rn(P.dr_std_thrust, dr_normal(P.dr_qtable, dr_field(r, 1)), 1.0f));
-                            az = __fmul_rn(az, __fmaf_rn(P.dr_std_thrust, dr_normal(P.dr_qtable, dr_field(r, 2)), 1.0f));
+                            thrust_noise(P, [=](int f) { return dr_normal(P.dr_qtable, dr_field(r, f)); }, ax, ay, az);
                         }
-                      if (PHYS) {
-                        // drone_physics_env.py:323-360 as a point mass (see the N <= 32 kernel below): per 1/240 s sub-step
-                        // speed clamp, thrust + 9.5 - 9.81 on z, Bullet's integrateVelocities -> applyDamping ->
-                        // integrateTransforms; v.w = this drone's damping factor
-                        const float h = DR ? c_dt : P.phys_h, f = v.w, gnet = P.phys_g_net;
-                        const float clamp_gate = __fmul_rn(__fmul_rn(c_vmax, c_vmax), 0.99999809265136719f /* 1 - 2^-19 */);
-#pragma unroll 1
-                        for (int sub = 0; sub < P.phys_substeps; ++sub) {
-                            if (sumsq_axis(v.x, v.y, v.z) > clamp_gate) {
-                                const float speed = norm1d<NORM>(v.x, v.y, v.z);
-                                if (speed > c_vmax) {
-                                    v.x = __fmul_rn(__fdiv_rn(v.x, speed), c_vmax);
-                                    v.y = __fmul_rn(__fdiv_rn(v.y, speed), c_vmax);
-                                    v.z = __fmul_rn(__fdiv_rn(v.z, speed), c_vmax);
-                                }
-                            }
-                            v.x = __fmul_rn(__fadd_rn(v.x, __fmul_rn(__fmul_rn(ax, c_amax), h)), f);
-                            v.y = __fmul_rn(__fadd_rn(v.y, __fmul_rn(__fmul_rn(ay, c_amax), h)), f);
-                            v.z = __fmul_rn(__fadd_rn(v.z, __fmul_rn(__fadd_rn(__fmul_rn(az, c_amax), gnet), h)), f);
-                            p.x = __fadd_rn(p.x, __fmul_rn(v.x, h));
-                            p.y = __fadd_rn(p.y, __fmul_rn(v.y, h));
-                            p.z = __fadd_rn(p.z, __fmul_rn(v.z, h));
-                        }
-                      } else {
-                        v.x = __fadd_rn(v.x, __fmul_rn(__fmul_rn(ax, c_amax), c_dt));
-                        v.y = __fadd_rn(v.y, __fmul_rn(__fmul_rn(ay, c_amax), c_dt));
-                        v.z = __fadd_rn(v.z, __fmul_rn(__fmul_rn(az, c_amax), c_dt));
-                        const float speed = norm1d<NORM>(v.x, v.y, v.z);  // _clip_speed (:179-183)
-                        if (!(speed <= c_vmax || speed < P.eps_speed)) {
-                            v.x = __fmul_rn(__fdiv_rn(v.x, speed), c_vmax);
-                            v.y = __fmul_rn(__fdiv_rn(v.y, speed), c_vmax);
-                            v.z = __fmul_rn(__fdiv_rn(v.z, speed), c_vmax);
-                        }
-                        p.x = __fadd_rn(p.x, __fmul_rn(v.x, c_dt));
-                        p.y = __fadd_rn(p.y, __fmul_rn(v.y, c_dt));
-                        p.z = __fadd_rn(p.z, __fmul_rn(v.z, c_dt));
-                      }
+                        if (PHYS) physics_substeps<NORM>(P, ax, ay, az, c_amax, c_vmax, DR ? c_dt : P.phys_h, p, v);
+                        else point_mass_step<NORM>(P, ax, ay, az, c_amax, c_vmax, c_dt, p.x, p.y, p.z, v.x, v.y, v.z);
                     }
                     // wall clip for ALL drones (:113-117); velocity is not zeroed at the wall (the physics env has no walls)
                     if (!PHYS) {
@@ -635,85 +582,30 @@ __global__ void __launch_bounds__(kThreadsPerCta, kMinBlocksPerSm) swarm_env_ker
             for (int el = 0; el < n_env; ++el) {
                 if (!((reset_envs >> el) & 1u)) continue;
                 const int renv = env0 + el;
-                const unsigned long long sh = P.rng[(long long)renv * 4 + 0], sl = P.rng[(long long)renv * 4 + 1];
-                const unsigned long long ih = P.rng[(long long)renv * 4 + 2], il = P.rng[(long long)renv * 4 + 3];
+                const Pcg64State rng = load_rng(P, renv);
                 double u_lo = P.rng_lo, u_range = P.rng_range;
                 if (DR) {
-                    // this episode's constants: 6 uniforms + an episode key from one counter per (env, reset)
-                    const unsigned ge = (unsigned)(P.env_index_base + renv);
-                    const uint4 ra = philox4x32_10(ge, (unsigned)sl, (unsigned)(sl >> 32), DR_CTR_EPISODE, P);
-                    const uint4 rb = philox4x32_10(ge, (unsigned)sl, (unsigned)(sl >> 32), DR_CTR_EPISODE + 1u, P);
-                    const double inv24 = 1.0 / 16777216.0;
-                    const double s_mass = __dadd_rn(P.dr_lo[0], __dmul_rn(P.dr_span[0], __dmul_rn((double)(ra.x >> 8), inv24)));
-                    const double s_acc = __dadd_rn(P.dr_lo[1], __dmul_rn(P.dr_span[1], __dmul_rn((double)(ra.y >> 8), inv24)));
-                    const double s_spd = __dadd_rn(P.dr_lo[2], __dmul_rn(P.dr_span[2], __dmul_rn((double)(ra.z >> 8), inv24)));
-                    const double s_dt = __dadd_rn(P.dr_lo[3], __dmul_rn(P.dr_span[3], __dmul_rn((double)(ra.w >> 8), inv24)));
-                    const double s_rad = __dadd_rn(P.dr_lo[4], __dmul_rn(P.dr_span[4], __dmul_rn((double)(rb.x >> 8), inv24)));
-                    const double s_wld = __dadd_rn(P.dr_lo[5], __dmul_rn(P.dr_span[5], __dmul_rn((double)(rb.y >> 8), inv24)));
-                    const double world = __dmul_rn(P.dr_world, s_wld);
-                    const double half_w = __dmul_rn(world, 0.5);
-                    u_lo = -half_w; u_range = __dsub_rn(half_w, -half_w);
-                    const float4 d0 = make_float4(__double2float_rn(__ddiv_rn(__dmul_rn(P.dr_max_accel, s_acc), s_mass)),
-                                                  __double2float_rn(__dmul_rn(P.dr_max_speed, s_spd)),
-                                                  __double2float_rn(__dmul_rn(P.dr_dt, s_dt)), __double2float_rn(half_w));
-                    float delay = 0.0f;  // this episode's control delay: 4th word of the second block
-                    if (P.dr_delay_count > 0) {
-                        const double uu = __dmul_rn((double)(rb.w >> 8), inv24);
-                        int pick = P.dr_delay_count - 1;
-                        for (int k = P.dr_delay_count - 1; k >= 0; --k)
-                            if (uu < P.dr_delay_cum[k]) pick = k;
-                        delay = (float)P.dr_delay_values[pick];
-                    }
-                    const float4 d1 = make_float4(__double2float_rn(__dadd_rn(P.dr_r_c, __dmul_rn(P.dr_r_o, s_rad))),
-                                                  __uint_as_float(rb.z), __double2float_rn(world), delay);
+                    const EpisodeDraw ep = draw_episode_constants(P, (unsigned)(P.env_index_base + renv), rng.sl);
+                    u_lo = ep.u_lo(); u_range = ep.u_range();
+                    float4 d0, d1;
+                    episode_params(P, ep, d0, d1);
                     if (lane == 0) {
                         P.dr_params[(long long)renv * 2 + 0] = d0;
                         P.dr_params[(long long)renv * 2 + 1] = d1;
                     }
                     if (lane_env_ok && e_l == el) {
-                        ekey = rb.z;
+                        ekey = ep.key;
                         c_vmax = d0.y;   // (physics: the observed velocity is clamped to this episode's max_speed)
                     }
                 }
-                for (int k = lane; k < P.n_draws; k += 32) {
-                    unsigned long long oh, ol;
-                    pcg_jump(P.jump[k + 1], sh, sl, ih, il, oh, ol);
-                    if (PHYS) {
-                        // drone_physics_env.py:207-242: per drone position (z >= 1), mass noise (cancels), damping
-                        // noise; obstacles (z >= 0.5); goal xy, one discarded draw, goal z in [0.5, 2]
-                        if (k < 5 * N) {
-                            const int dr_ = k / 5, c5 = k - 5 * dr_;
-                            if (c5 < 3) {
-                                float val = pcg_uniform_f32(oh, ol, u_lo, u_range);
-                                if (c5 == 2) val = fmaxf(val, 1.0f);
-                                reinterpret_cast<float*>(tab_pos + el * N + dr_)[c5] = val;
-                            } else if (c5 == 4) {
-                                const double c_lin = __dmul_rn(0.5, pcg_uniform_f64(oh, ol, 0.8, 1.2 - 0.8));
-                                reinterpret_cast<float*>(tab_vel + el * N + dr_)[3] = __double2float_rn(phys_damp_factor(c_lin));
-                            }
-                        } else if (k < 5 * N + 3 * M) {
-                            const int kk = k - 5 * N, m_ = kk / 3, c3 = kk - 3 * m_;
-                            float val = pcg_uniform_f32(oh, ol, u_lo, u_range);
-                            if (c3 == 2) val = fmaxf(val, 0.5f);
-                            reinterpret_cast<float*>(tab_obst + el * P.m_pad + m_)[c3] = val;
-                        } else {
-                            const int g_ = k - 5 * N - 3 * M;
-                            if (g_ < 2) reinterpret_cast<float*>(tab_goal + el)[g_] = pcg_uniform_f32(oh, ol, u_lo, u_range);
-                            else if (g_ == 3) reinterpret_cast<float*>(tab_goal + el)[2] = pcg_uniform_f32(oh, ol, 0.5, 2.0 - 0.5);
-                        }
-                        continue;
-                    }
-                    const float val = pcg_uniform_f32(oh, ol, u_lo, u_range);
-                    // draw order: positions (N,3) -> goal (3,) -> obstacles (M,3)
-                    if (k < 3 * N) {
-                        reinterpret_cast<float*>(tab_pos + el * N + k / 3)[k % 3] = val;
-                    } else if (k < 3 * N + 3) {
-                        reinterpret_cast<float*>(tab_goal + el)[k - 3 * N] = val;
-                    } else {
-                        const int kk = k - 3 * N - 3;
-                        reinterpret_cast<float*>(tab_obst + el * P.m_pad + kk / 3)[kk % 3] = val;
-                    }
-                }
+                auto pos = [=](int j) { return reinterpret_cast<float*>(tab_pos + el * N + j); };
+                auto goal = [=]() { return reinterpret_cast<float*>(tab_goal + el); };
+                auto obst = [=](int m) { return reinterpret_cast<float*>(tab_obst + el * P.m_pad + m); };
+                if (PHYS)
+                    reset_env_physics_draws<1>(P, lane, N, M, rng, u_lo, u_range, pos,
+                                               [=](int j) { return reinterpret_cast<float*>(tab_vel + el * N + j); }, goal, obst);
+                else
+                    reset_env_draws<1>(P, lane, N, rng, u_lo, u_range, pos, goal, obst);
                 for (int k = lane; k < N; k += 32) {
                     reinterpret_cast<float*>(tab_pos + el * N + k)[3] = 1.0f;
                     float* tv = reinterpret_cast<float*>(tab_vel + el * N + k);
@@ -721,12 +613,7 @@ __global__ void __launch_bounds__(kThreadsPerCta, kMinBlocksPerSm) swarm_env_ker
                     if (!PHYS) tv[3] = 0.f;  // (physics: .w holds this drone's new damping factor)
                 }
                 if (lane == 0) {
-                    unsigned long long oh, ol;
-                    pcg_jump(P.jump[P.n_draws], sh, sl, ih, il, oh, ol);
-                    P.rng[(long long)renv * 4 + 0] = oh;
-                    P.rng[(long long)renv * 4 + 1] = ol;
-                    P.step_count[renv] = 0;
-                    P.ep_return[renv] = 0.0f;
+                    reset_env_finish(P, renv, rng);
                     reinterpret_cast<float*>(tab_goal + el)[3] = 0.0f;
                 }
                 for (int k = lane; k < M; k += 32) reinterpret_cast<float*>(tab_obst + el * P.m_pad + k)[3] = 0.0f;
@@ -1052,95 +939,25 @@ __global__ void __launch_bounds__(kThreadsPerCta, kMinBlocksPerSm) swarm_env_ker
             // =========================== phase A: integrate (:98-118) ===========================
             prev_d = norm1d<NORM>(__fsub_rn(gx, p.x), __fsub_rn(gy, p.y), __fsub_rn(gz, p.z));  // :98-101
             if (PHYS) {
-                // drone_physics_env.py:323-360 as a point mass: per 1/240 s sub-step speed clamp, thrust
-                // (action neither clipped nor cast; the mass cancels) + 9.5 - 9.81 on z, Bullet's
-                // integrateVelocities -> applyDamping -> integrateTransforms; v.w = this drone's damping factor
                 if (alive) {
                     // DR on top (DESIGN.md 9): the episode's sub-step length rides in c_dt; control delay and thrust
                     // noise act on the command, which is then held for the whole step (no clip: :336)
-                    if (DR && P.dr_delay_hist > 0) {
-                        const int H = P.dr_delay_hist;
-                        float* ring = P.act_hist + (long long)env * H * N * 3 + i * 3;
-                        const float sx = ax, sy = ay, sz = az;
-                        if (ctrl_delay > 0) {
-                            if (sc < ctrl_delay) {
-                                ax = 0.f; ay = 0.f; az = 0.f;
-                            } else {
-                                const float* hp = ring + (long long)((sc - ctrl_delay) % H) * N * 3;
-                                ax = hp[0]; ay = hp[1]; az = hp[2];
-                            }
-                        }
-                        float* wp = ring + (long long)(sc % H) * N * 3;
-                        wp[0] = sx; wp[1] = sy; wp[2] = sz;
-                    }
+                    if (DR && P.dr_delay_hist > 0) delayed_command(P, env, N, i, sc, ctrl_delay, ax, ay, az);
                     if (DR) {
                         const uint4 r = philox4x32_7(genv, ekey, (unsigned)sc, (unsigned)i | (DR_STREAM_A << 16), P);
-                        ax = __fmul_rn(ax, __fmaf_rn(P.dr_std_thrust, dr_normal(P.dr_qtable, dr_field(r, 0)), 1.0f));
-                        ay = __fmul_rn(ay, __fmaf_rn(P.dr_std_thrust, dr_normal(P.dr_qtable, dr_field(r, 1)), 1.0f));
-                        az = __fmul_rn(az, __fmaf_rn(P.dr_std_thrust, dr_normal(P.dr_qtable, dr_field(r, 2)), 1.0f));
+                        thrust_noise(P, [=](int f) { return dr_normal(P.dr_qtable, dr_field(r, f)); }, ax, ay, az);
                     }
-                    const float h = DR ? c_dt : P.phys_h, f = v.w, gnet = P.phys_g_net;
-                    // |v| can exceed max_speed only if the plain float32 sum of squares (within 2^-22 of the exact
-                    // one, like the reference's norm) comes within 2^-19 of max_speed^2: the exact norm -- float64
-                    // accumulate + IEEE sqrt, 24 times per step -- is evaluated only then (NaN compares false on
-                    // both sides)
-                    const float clamp_gate = __fmul_rn(__fmul_rn(c_vmax, c_vmax), 0.99999809265136719f /* 1 - 2^-19 */);
-#pragma unroll 1
-                    for (int sub = 0; sub < P.phys_substeps; ++sub) {
-                        if (sumsq_axis(v.x, v.y, v.z) > clamp_gate) {
-                            const float speed = norm1d<NORM>(v.x, v.y, v.z);
-                            if (speed > c_vmax) {
-                                v.x = __fmul_rn(__fdiv_rn(v.x, speed), c_vmax);
-                                v.y = __fmul_rn(__fdiv_rn(v.y, speed), c_vmax);
-                                v.z = __fmul_rn(__fdiv_rn(v.z, speed), c_vmax);
-                            }
-                        }
-                        v.x = __fmul_rn(__fadd_rn(v.x, __fmul_rn(__fmul_rn(ax, c_amax), h)), f);
-                        v.y = __fmul_rn(__fadd_rn(v.y, __fmul_rn(__fmul_rn(ay, c_amax), h)), f);
-                        v.z = __fmul_rn(__fadd_rn(v.z, __fmul_rn(__fadd_rn(__fmul_rn(az, c_amax), gnet), h)), f);
-                        p.x = __fadd_rn(p.x, __fmul_rn(v.x, h));
-                        p.y = __fadd_rn(p.y, __fmul_rn(v.y, h));
-                        p.z = __fadd_rn(p.z, __fmul_rn(v.z, h));
-                    }
+                    physics_substeps<NORM>(P, ax, ay, az, c_amax, c_vmax, DR ? c_dt : P.phys_h, p, v);
                 }
             } else if (alive) {
-                if (DR && P.dr_delay_hist > 0) {
-                    // control delay: apply the command submitted ctrl_delay steps ago (zero while the episode is
-                    // younger), then file the one submitted now in ring slot step_count % H
-                    const int H = P.dr_delay_hist;
-                    float* ring = P.act_hist + (long long)env * H * N * 3 + i * 3;
-                    const float sx = ax, sy = ay, sz = az;
-                    if (ctrl_delay > 0) {
-                        if (sc < ctrl_delay) {
-                            ax = 0.f; ay = 0.f; az = 0.f;
-                        } else {
-                            const float* hp = ring + (long long)((sc - ctrl_delay) % H) * N * 3;
-                            ax = hp[0]; ay = hp[1]; az = hp[2];
-                        }
-                    }
-                    float* wp = ring + (long long)(sc % H) * N * 3;
-                    wp[0] = sx; wp[1] = sy; wp[2] = sz;
-                }
+                if (DR && P.dr_delay_hist > 0) delayed_command(P, env, N, i, sc, ctrl_delay, ax, ay, az);
                 ax = clipf(ax, -1.0f, 1.0f); ay = clipf(ay, -1.0f, 1.0f); az = clipf(az, -1.0f, 1.0f);
                 nan_act = !(ax == ax && ay == ay && az == az);   // (np.clip lets NaN through; counted below)
-                if (DR) {  // thrust noise: a <- a * (1 + sigma z), one normal per axis
+                if (DR) {
                     const uint4 r = philox4x32_7(genv, ekey, (unsigned)sc, (unsigned)i | (DR_STREAM_A << 16), P);
-                    ax = __fmul_rn(ax, __fmaf_rn(P.dr_std_thrust, dr_normal(P.dr_qtable, dr_field(r, 0)), 1.0f));
-                    ay = __fmul_rn(ay, __fmaf_rn(P.dr_std_thrust, dr_normal(P.dr_qtable, dr_field(r, 1)), 1.0f));
-                    az = __fmul_rn(az, __fmaf_rn(P.dr_std_thrust, dr_normal(P.dr_qtable, dr_field(r, 2)), 1.0f));
+                    thrust_noise(P, [=](int f) { return dr_normal(P.dr_qtable, dr_field(r, f)); }, ax, ay, az);
                 }
-                v.x = __fadd_rn(v.x, __fmul_rn(__fmul_rn(ax, c_amax), c_dt));
-                v.y = __fadd_rn(v.y, __fmul_rn(__fmul_rn(ay, c_amax), c_dt));
-                v.z = __fadd_rn(v.z, __fmul_rn(__fmul_rn(az, c_amax), c_dt));
-                const float speed = norm1d<NORM>(v.x, v.y, v.z);  // _clip_speed (:179-183)
-                if (!(speed <= c_vmax || speed < P.eps_speed)) {
-                    v.x = __fmul_rn(__fdiv_rn(v.x, speed), c_vmax);
-                    v.y = __fmul_rn(__fdiv_rn(v.y, speed), c_vmax);
-                    v.z = __fmul_rn(__fdiv_rn(v.z, speed), c_vmax);
-                }
-                p.x = __fadd_rn(p.x, __fmul_rn(v.x, c_dt));
-                p.y = __fadd_rn(p.y, __fmul_rn(v.y, c_dt));
-                p.z = __fadd_rn(p.z, __fmul_rn(v.z, c_dt));
+                point_mass_step<NORM>(P, ax, ay, az, c_amax, c_vmax, c_dt, p.x, p.y, p.z, v.x, v.y, v.z);
             }
             if (PHYS) nan_act = alive && !(ax == ax && ay == ay && az == az);   // (the physics env does not clip)
             {   // NaN-action guard counter (rare: the vote is all a clean step pays)
@@ -1171,91 +988,31 @@ __global__ void __launch_bounds__(kThreadsPerCta, kMinBlocksPerSm) swarm_env_ker
             for (int el = 0; el < n_env; ++el) {
                 if (!((reset_envs >> el) & 1u)) continue;
                 const int renv = env0 + el;
-                const unsigned long long sh = P.rng[(long long)renv * 4 + 0], sl = P.rng[(long long)renv * 4 + 1];
-                const unsigned long long ih = P.rng[(long long)renv * 4 + 2], il = P.rng[(long long)renv * 4 + 3];
+                const Pcg64State rng = load_rng(P, renv);
                 double u_lo = P.rng_lo, u_range = P.rng_range;
                 if (DR) {
-                    // this episode's constants: 6 uniforms + an episode key from one counter per (env, reset)
-                    const unsigned ge = (unsigned)(P.env_index_base + renv);
-                    const uint4 ra = philox4x32_10(ge, (unsigned)sl, (unsigned)(sl >> 32), DR_CTR_EPISODE, P);
-                    const uint4 rb = philox4x32_10(ge, (unsigned)sl, (unsigned)(sl >> 32), DR_CTR_EPISODE + 1u, P);
-                    const double inv24 = 1.0 / 16777216.0;
-                    const double s_mass = __dadd_rn(P.dr_lo[0], __dmul_rn(P.dr_span[0], __dmul_rn((double)(ra.x >> 8), inv24)));
-                    const double s_acc = __dadd_rn(P.dr_lo[1], __dmul_rn(P.dr_span[1], __dmul_rn((double)(ra.y >> 8), inv24)));
-                    const double s_spd = __dadd_rn(P.dr_lo[2], __dmul_rn(P.dr_span[2], __dmul_rn((double)(ra.z >> 8), inv24)));
-                    const double s_dt = __dadd_rn(P.dr_lo[3], __dmul_rn(P.dr_span[3], __dmul_rn((double)(ra.w >> 8), inv24)));
-                    const double s_rad = __dadd_rn(P.dr_lo[4], __dmul_rn(P.dr_span[4], __dmul_rn((double)(rb.x >> 8), inv24)));
-                    const double s_wld = __dadd_rn(P.dr_lo[5], __dmul_rn(P.dr_span[5], __dmul_rn((double)(rb.y >> 8), inv24)));
-                    const double world = __dmul_rn(P.dr_world, s_wld);
-                    const double half_w = __dmul_rn(world, 0.5);
-                    u_lo = -half_w; u_range = __dsub_rn(half_w, -half_w);
+                    const EpisodeDraw ep = draw_episode_constants(P, (unsigned)(P.env_index_base + renv), rng.sl);
+                    u_lo = ep.u_lo(); u_range = ep.u_range();
+                    float4 d0, d1;
+                    episode_params(P, ep, d0, d1);
                     if (lane == 0) {
-                        const float4 d0 = make_float4(__double2float_rn(__ddiv_rn(__dmul_rn(P.dr_max_accel, s_acc), s_mass)),
-                                                      __double2float_rn(__dmul_rn(P.dr_max_speed, s_spd)),
-                                                      __double2float_rn(__dmul_rn(P.dr_dt, s_dt)), __double2float_rn(half_w));
-                        float delay = 0.0f;  // this episode's control delay: 4th word of the second block
-                        if (P.dr_delay_count > 0) {
-                            const double uu = __dmul_rn((double)(rb.w >> 8), inv24);
-                            int pick = P.dr_delay_count - 1;
-                            for (int k = P.dr_delay_count - 1; k >= 0; --k)
-                                if (uu < P.dr_delay_cum[k]) pick = k;
-                            delay = (float)P.dr_delay_values[pick];
-                        }
-                        const float4 d1 = make_float4(__double2float_rn(__dadd_rn(P.dr_r_c, __dmul_rn(P.dr_r_o, s_rad))),
-                                                      __uint_as_float(rb.z), __double2float_rn(world), delay);
                         P.dr_params[(long long)renv * 2 + 0] = d0;
                         P.dr_params[(long long)renv * 2 + 1] = d1;
                     }
                     if (lane_ok && e_l == el) {
-                        c_amax = __double2float_rn(__ddiv_rn(__dmul_rn(P.dr_max_accel, s_acc), s_mass));
-                        c_vmax = __double2float_rn(__dmul_rn(P.dr_max_speed, s_spd));
-                        c_dt = __double2float_rn(__dmul_rn(P.dr_dt, s_dt));
-                        c_bound = __double2float_rn(half_w);
-                        c_thr_obst = __double2float_rn(__dadd_rn(P.dr_r_c, __dmul_rn(P.dr_r_o, s_rad)));
-                        ekey = rb.z;
+                        c_amax = d0.x; c_vmax = d0.y; c_dt = d0.z; c_bound = d0.w;
+                        c_thr_obst = d1.x; ekey = ep.key;
                         sc_obs = 0;
                     }
                 }
-#pragma unroll 1
-                for (int k = lane; k < P.n_draws; k += 32) {
-                    unsigned long long oh, ol;
-                    pcg_jump(P.jump[k + 1], sh, sl, ih, il, oh, ol);
-                    if (PHYS) {
-                        // drone_physics_env.py:207-242: per drone position (z >= 1), mass noise (cancels), damping
-                        // noise; obstacles (z >= 0.5); goal xy, one discarded draw, goal z in [0.5, 2]
-                        if (k < 5 * N) {
-                            const int dr_ = k / 5, c5 = k - 5 * dr_;
-                            if (c5 < 3) {
-                                float val = pcg_uniform_f32(oh, ol, u_lo, u_range);
-                                if (c5 == 2) val = fmaxf(val, 1.0f);
-                                reinterpret_cast<float*>(tab_pos + el * N + dr_)[c5] = val;
-                            } else if (c5 == 4) {
-                                const double c_lin = __dmul_rn(0.5, pcg_uniform_f64(oh, ol, 0.8, 1.2 - 0.8));
-                                reinterpret_cast<float*>(tab_vel + el * N + dr_)[3] = __double2float_rn(phys_damp_factor(c_lin));
-                            }
-                        } else if (k < 5 * N + 3 * M) {
-                            const int kk = k - 5 * N, m_ = kk / 3, c3 = kk - 3 * m_;
-                            float val = pcg_uniform_f32(oh, ol, u_lo, u_range);
-                            if (c3 == 2) val = fmaxf(val, 0.5f);
-                            reinterpret_cast<float*>(tab_obst + el * P.m_pad + m_)[c3] = val;
-                        } else {
-                            const int g_ = k - 5 * N - 3 * M;
-                            if (g_ < 2) reinterpret_cast<float*>(tab_goal + el)[g_] = pcg_uniform_f32(oh, ol, u_lo, u_range);
-                            else if (g_ == 3) reinterpret_cast<float*>(tab_goal + el)[2] = pcg_uniform_f32(oh, ol, 0.5, 2.0 - 0.5);
-                        }
-                        continue;
-                    }
-                    const float val = pcg_uniform_f32(oh, ol, u_lo, u_range);
-                    // draw order: positions (N,3) -> goal (3,) -> obstacles (M,3)
-                    if (k < 3 * N) {
-                        reinterpret_cast<float*>(tab_pos + el * N + k / 3)[k % 3] = val;
-                    } else if (k < 3 * N + 3) {
-                        reinterpret_cast<float*>(tab_goal + el)[k - 3 * N] = val;
-                    } else {
-                        const int kk = k - 3 * N - 3;
-                        reinterpret_cast<float*>(tab_obst + el * P.m_pad + kk / 3)[kk % 3] = val;
-                    }
-                }
+                auto pos = [=](int j) { return reinterpret_cast<float*>(tab_pos + el * N + j); };
+                auto goal = [=]() { return reinterpret_cast<float*>(tab_goal + el); };
+                auto obst = [=](int m) { return reinterpret_cast<float*>(tab_obst + el * P.m_pad + m); };
+                if (PHYS)
+                    reset_env_physics_draws<1>(P, lane, N, M, rng, u_lo, u_range, pos,
+                                               [=](int j) { return reinterpret_cast<float*>(tab_vel + el * N + j); }, goal, obst);
+                else
+                    reset_env_draws<1>(P, lane, N, rng, u_lo, u_range, pos, goal, obst);
                 if (lane < N) {
                     reinterpret_cast<float*>(tab_pos + el * N + lane)[3] = 1.0f;
                     float* tv = reinterpret_cast<float*>(tab_vel + el * N + lane);
@@ -1263,12 +1020,7 @@ __global__ void __launch_bounds__(kThreadsPerCta, kMinBlocksPerSm) swarm_env_ker
                     if (!PHYS) tv[3] = 0.f;  // (physics: .w already holds this drone's damping factor)
                 }
                 if (lane == 0) {
-                    unsigned long long oh, ol;
-                    pcg_jump(P.jump[P.n_draws], sh, sl, ih, il, oh, ol);
-                    P.rng[(long long)renv * 4 + 0] = oh;
-                    P.rng[(long long)renv * 4 + 1] = ol;
-                    P.step_count[renv] = 0;
-                    P.ep_return[renv] = 0.0f;
+                    reset_env_finish(P, renv, rng);
                     reinterpret_cast<float*>(tab_goal + el)[3] = 0.0f;
                 }
                 for (int k = lane; k < M; k += 32) reinterpret_cast<float*>(tab_obst + el * P.m_pad + k)[3] = 0.0f;

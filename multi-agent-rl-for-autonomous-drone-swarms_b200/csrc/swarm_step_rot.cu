@@ -407,45 +407,14 @@ __global__ void __launch_bounds__(rot_warps(NT, DRM != 0) * 32, rot_min_blocks(N
                 // =========================== integrate (:98-118) ===========================
                 prev_d = norm1d<0>(__fsub_rn(gx, p.x), __fsub_rn(gy, p.y), __fsub_rn(gz, p.z));  // :98-101
                 if (alive) {
-                    if (DRM == 2 && P.dr_delay_hist > 0) {
-                        // control delay: apply the command submitted ctrl_delay steps ago (zero while the episode
-                        // is younger), then file the one submitted now in ring slot step_count % H
-                        const int H = P.dr_delay_hist;
-                        float* ring = P.act_hist + ((long long)env * H * N + i) * 3;
-                        const float sx = ax, sy = ay, sz = az;
-                        const int slot_w = (int)((unsigned)sc % (unsigned)H);
-                        if (ctrl_delay > 0) {
-                            if (sc < ctrl_delay) {
-                                ax = 0.f; ay = 0.f; az = 0.f;
-                            } else {  // (sc - ctrl_delay) % H without a second division: ctrl_delay <= H
-                                const int slot_r = slot_w - ctrl_delay + (slot_w < ctrl_delay ? H : 0);
-                                const float* hp = ring + slot_r * (N * 3);
-                                ax = hp[0]; ay = hp[1]; az = hp[2];
-                            }
-                        }
-                        float* wp = ring + slot_w * (N * 3);
-                        wp[0] = sx; wp[1] = sy; wp[2] = sz;
-                    }
+                    if (DRM == 2 && P.dr_delay_hist > 0) delayed_command(P, env, N, i, sc, ctrl_delay, ax, ay, az);
                     ax = clipf(ax, -1.0f, 1.0f); ay = clipf(ay, -1.0f, 1.0f); az = clipf(az, -1.0f, 1.0f);
                     nan_act = !(ax == ax && ay == ay && az == az);   // (np.clip lets NaN through; counted, see below)
-                    if (DR) {  // thrust noise: a <- a * (1 + sigma z), one normal per axis
+                    if (DR) {
                         rA = philox4x32_7(genv, ekey, (unsigned)sc, (unsigned)i | (DR_STREAM_A << 16), P);
-                        ax = __fmul_rn(ax, __fmaf_rn(P.dr_std_thrust, dr_normal_off(qtab, dr_field_off(rA, 0)), 1.0f));
-                        ay = __fmul_rn(ay, __fmaf_rn(P.dr_std_thrust, dr_normal_off(qtab, dr_field_off(rA, 1)), 1.0f));
-                        az = __fmul_rn(az, __fmaf_rn(P.dr_std_thrust, dr_normal_off(qtab, dr_field_off(rA, 2)), 1.0f));
+                        thrust_noise(P, [=](int f) { return dr_normal_off(qtab, dr_field_off(rA, f)); }, ax, ay, az);
                     }
-                    v.x = __fadd_rn(v.x, __fmul_rn(__fmul_rn(ax, c_amax), c_dt));
-                    v.y = __fadd_rn(v.y, __fmul_rn(__fmul_rn(ay, c_amax), c_dt));
-                    v.z = __fadd_rn(v.z, __fmul_rn(__fmul_rn(az, c_amax), c_dt));
-                    const float speed = norm1d<0>(v.x, v.y, v.z);  // _clip_speed (:179-183)
-                    if (!(speed <= c_vmax || speed < P.eps_speed)) {
-                        v.x = __fmul_rn(__fdiv_rn(v.x, speed), c_vmax);
-                        v.y = __fmul_rn(__fdiv_rn(v.y, speed), c_vmax);
-                        v.z = __fmul_rn(__fdiv_rn(v.z, speed), c_vmax);
-                    }
-                    p.x = __fadd_rn(p.x, __fmul_rn(v.x, c_dt));
-                    p.y = __fadd_rn(p.y, __fmul_rn(v.y, c_dt));
-                    p.z = __fadd_rn(p.z, __fmul_rn(v.z, c_dt));
+                    point_mass_step<0>(P, ax, ay, az, c_amax, c_vmax, c_dt, p.x, p.y, p.z, v.x, v.y, v.z);
                 }
                 {   // NaN-action guard counter (rare: the vote is all a clean step pays)
                     const unsigned nan_m = __ballot_sync(FULL_MASK, nan_act);
@@ -458,47 +427,18 @@ __global__ void __launch_bounds__(rot_warps(NT, DRM != 0) * 32, rot_min_blocks(N
             } else {
                 __syncwarp();  // every lane is done with the previous item's tables
                 // ================================ reset (:65-80) ================================
-                // draw order of env.reset(): positions (N,3) -> goal (3,) -> obstacles (M,3), each
-                // rng.uniform(-W/2, W/2) in float64 then float32; 32 lanes draw in parallel by PCG64 jump-ahead
 #pragma unroll 1
                 for (int el = 0; el < n_env; ++el) {
                     if (!((reset_envs >> el) & 1u)) continue;
                     const int renv = env0 + el;
-                    const unsigned long long sh = P.rng[(long long)renv * 4 + 0], sl = P.rng[(long long)renv * 4 + 1];
-                    const unsigned long long ih = P.rng[(long long)renv * 4 + 2], il = P.rng[(long long)renv * 4 + 3];
+                    const Pcg64State rng = load_rng(P, renv);
                     double u_lo = P.rng_lo, u_range = P.rng_range;
                     if (DR) {
-                        // this episode's constants: 6 uniforms + an episode key from one counter per (env, reset)
-                        const unsigned ge = (unsigned)(P.env_index_base + renv);
-                        const uint4 ra = philox4x32_10(ge, (unsigned)sl, (unsigned)(sl >> 32), DR_CTR_EPISODE, P);
-                        const uint4 rb = philox4x32_10(ge, (unsigned)sl, (unsigned)(sl >> 32), DR_CTR_EPISODE + 1u, P);
-                        const double inv24 = 1.0 / 16777216.0;
-                        const double s_mass = __dadd_rn(P.dr_lo[0], __dmul_rn(P.dr_span[0], __dmul_rn((double)(ra.x >> 8), inv24)));
-                        const double s_acc = __dadd_rn(P.dr_lo[1], __dmul_rn(P.dr_span[1], __dmul_rn((double)(ra.y >> 8), inv24)));
-                        const double s_spd = __dadd_rn(P.dr_lo[2], __dmul_rn(P.dr_span[2], __dmul_rn((double)(ra.z >> 8), inv24)));
-                        const double s_dt = __dadd_rn(P.dr_lo[3], __dmul_rn(P.dr_span[3], __dmul_rn((double)(ra.w >> 8), inv24)));
-                        const double s_rad = __dadd_rn(P.dr_lo[4], __dmul_rn(P.dr_span[4], __dmul_rn((double)(rb.x >> 8), inv24)));
-                        const double s_wld = __dadd_rn(P.dr_lo[5], __dmul_rn(P.dr_span[5], __dmul_rn((double)(rb.y >> 8), inv24)));
-                        const double world = __dmul_rn(P.dr_world, s_wld);
-                        const double half_w = __dmul_rn(world, 0.5);
-                        u_lo = -half_w; u_range = __dsub_rn(half_w, -half_w);
+                        const EpisodeDraw ep = draw_episode_constants(P, (unsigned)(P.env_index_base + renv), rng.sl);
+                        u_lo = ep.u_lo(); u_range = ep.u_range();
                         if (lane == 0) {
-                            float delay = 0.0f;  // this episode's control delay: 4th word of the second block
-                            if (P.dr_delay_count > 0) {
-                                const double uu = __dmul_rn((double)(rb.w >> 8), inv24);
-                                int pick = P.dr_delay_count - 1;
-#pragma unroll 1
-                                for (int k = P.dr_delay_count - 1; k >= 0; --k)
-                                    if (uu < P.dr_delay_cum[k]) pick = k;
-                                delay = (float)P.dr_delay_values[pick];
-                            }
-                            const float4 d0 =
-                                make_float4(__double2float_rn(__ddiv_rn(__dmul_rn(P.dr_max_accel, s_acc), s_mass)),
-                                            __double2float_rn(__dmul_rn(P.dr_max_speed, s_spd)),
-                                            __double2float_rn(__dmul_rn(P.dr_dt, s_dt)), __double2float_rn(half_w));
-                            const float4 d1 =
-                                make_float4(__double2float_rn(__dadd_rn(P.dr_r_c, __dmul_rn(P.dr_r_o, s_rad))),
-                                            __uint_as_float(rb.z), __double2float_rn(world), delay);
+                            float4 d0, d1;
+                            episode_params(P, ep, d0, d1);
                             P.dr_params[(long long)renv * 2 + 0] = d0;
                             P.dr_params[(long long)renv * 2 + 1] = d1;
                             if (kFused) {   // (resident mode reads them from here on the next step)
@@ -506,29 +446,15 @@ __global__ void __launch_bounds__(rot_warps(NT, DRM != 0) * 32, rot_min_blocks(N
                                 drp[0] = d0; drp[1] = d1;
                             }
                         }
-                        if (e_l == el) ekey = rb.z;  // (the dynamics constants are not needed to observe)
+                        if (e_l == el) ekey = ep.key;  // (the dynamics constants are not needed to observe)
                     }
-#pragma unroll (kFused ? 1 : 4)
-                    for (int k = lane; k < P.n_draws; k += 32) {
-                        unsigned long long oh, ol;
-                        pcg_jump(P.jump[k + 1], sh, sl, ih, il, oh, ol);
-                        const float val = pcg_uniform_f32(oh, ol, u_lo, u_range);
-                        if (k < 3 * N) {
-                            reinterpret_cast<float*>(tab2 + 2 * el * N + k / 3)[k % 3] = val;
-                        } else if (k < 3 * N + 3) {
-                            reinterpret_cast<float*>(tgoal + el)[k - 3 * N] = val;
-                        } else {
-                            const int kk = k - 3 * N - 3;
-                            reinterpret_cast<float*>(tobs_all + el * M + kk / 3)[kk % 3] = val;
-                        }
-                    }
+                    reset_env_draws<kFused ? 1 : 4>(
+                        P, lane, N, rng, u_lo, u_range,
+                        [=](int j) { return reinterpret_cast<float*>(tab2 + 2 * el * N + j); },
+                        [=]() { return reinterpret_cast<float*>(tgoal + el); },
+                        [=](int m) { return reinterpret_cast<float*>(tobs_all + el * M + m); });
                     if (lane == 0) {
-                        unsigned long long oh, ol;
-                        pcg_jump(P.jump[P.n_draws], sh, sl, ih, il, oh, ol);
-                        P.rng[(long long)renv * 4 + 0] = oh;
-                        P.rng[(long long)renv * 4 + 1] = ol;
-                        P.step_count[renv] = 0;
-                        P.ep_return[renv] = 0.0f;
+                        reset_env_finish(P, renv, rng);
                         reinterpret_cast<float*>(tgoal + el)[3] = 0.0f;
                     }
                     for (int k = lane; k < M; k += 32)  // obstacle index in .w (one-LOP3 keys, as in the step launch)
@@ -1006,32 +932,14 @@ __global__ void __launch_bounds__(rot_warps(NT, DRM != 0) * 32, rot_min_blocks(N
             const unsigned out_envs = step_pass() ? (((1u << n_env) - 1u) & ~redraw_envs) : reset_envs;
             if (out_envs != 0u) {
                 if (lane_ok && (!kFused || ((out_envs >> e_l) & 1u))) {
-                    float* row = srow;
                     const float4 t0 = tab2[2 * e_base + nj[0]], t1 = tab2[2 * e_base + nj[1]], t2 = tab2[2 * e_base + nj[2]];
                     const float4 b0 = tobs[om[0]], b1 = tobs[om[1]], b2 = tobs[om[2]], b3 = tobs[om[3]];
                     if (DR) {  // sensor noise of the observed state (step_count sc + 1): the block of counter sc
                         if (!step_pass() || !alive)  // (an active drone drew this block for its thrust already)
                             rA = philox4x32_7(genv, ekey, (unsigned)sc, (unsigned)i | (DR_STREAM_A << 16), P);
                     }
-                    auto noisy = [&](float x, float sigma, unsigned idx) {
-                        return DR ? __fmaf_rn(sigma, dr_normal_off(qtab, idx), x) : x;
-                    };
-                    row[0] = noisy(p.x, P.dr_std_pos, dr_field_off(rA, 3)); row[1] = noisy(p.y, P.dr_std_pos, dr_field_off(rA, 4));
-                    row[2] = noisy(p.z, P.dr_std_pos, dr_field_off(rA, 5));
-                    row[3] = noisy(v.x, P.dr_std_vel, dr_field_off(rA, 6)); row[4] = noisy(v.y, P.dr_std_vel, dr_field_off(rA, 7));
-                    row[5] = noisy(v.z, P.dr_std_vel, dr_field_off(rA, 8));
-                    row[6] = __fsub_rn(gx, p.x); row[7] = __fsub_rn(gy, p.y); row[8] = __fsub_rn(gz, p.z);
-                    row[9] = __fsub_rn(t0.x, p.x); row[10] = __fsub_rn(t0.y, p.y); row[11] = __fsub_rn(t0.z, p.z); row[12] = nd[0];
-                    row[13] = __fsub_rn(t1.x, p.x); row[14] = __fsub_rn(t1.y, p.y); row[15] = __fsub_rn(t1.z, p.z); row[16] = nd[1];
-                    row[17] = __fsub_rn(t2.x, p.x); row[18] = __fsub_rn(t2.y, p.y); row[19] = __fsub_rn(t2.z, p.z); row[20] = nd[2];
-                    row[21] = __fsub_rn(b0.x, p.x); row[22] = __fsub_rn(b0.y, p.y); row[23] = __fsub_rn(b0.z, p.z);
-                    row[24] = noisy(od[0], P.dr_std_obst, dr_field_off(rA, 9));
-                    row[25] = __fsub_rn(b1.x, p.x); row[26] = __fsub_rn(b1.y, p.y); row[27] = __fsub_rn(b1.z, p.z);
-                    row[28] = noisy(od[1], P.dr_std_obst, dr_field_off(rA, 10));
-                    row[29] = __fsub_rn(b2.x, p.x); row[30] = __fsub_rn(b2.y, p.y); row[31] = __fsub_rn(b2.z, p.z);
-                    row[32] = noisy(od[2], P.dr_std_obst, dr_field_off(rA, 11));
-                    row[33] = __fsub_rn(b3.x, p.x); row[34] = __fsub_rn(b3.y, p.y); row[35] = __fsub_rn(b3.z, p.z);
-                    row[36] = noisy(od[3], P.dr_std_obst, dr_field_off(rA, 12));
+                    observe_row_k3s4<DR>(P, srow, p.x, p.y, p.z, v.x, v.y, v.z, gx, gy, gz, t0, t1, t2, nd, b0, b1, b2, b3, od,
+                                         [=](int f) { return dr_normal_off(qtab, dr_field_off(rA, f)); });
                 }
                 fence_async_smem();  // generic-proxy tile writes -> visible to the bulk-copy engine
                 __syncwarp();

@@ -198,43 +198,14 @@ swarm_step_rotx_kernel(const DevParams P) {
                 px[s] = p.x; py[s] = p.y; pz[s] = p.z;
                 prev_d[s] = norm1d<0>(__fsub_rn(gx, p.x), __fsub_rn(gy, p.y), __fsub_rn(gz, p.z));  // :98-101
                 if (alive[s]) {  // integrate (:103-111)
-                    if (DR && P.dr_delay_hist > 0) {
-                        // control delay: apply the command submitted ctrl_delay steps ago (zero while the episode is
-                        // younger), then file the one submitted now in ring slot step_count % H
-                        const int H = P.dr_delay_hist;
-                        float* ring = P.act_hist + ((long long)env * H * N + (s * 32 + lane)) * 3;
-                        const float sx = ax, sy = ay, sz = az;
-                        if (ctrl_delay > 0) {
-                            if (sc < ctrl_delay) {
-                                ax = 0.f; ay = 0.f; az = 0.f;
-                            } else {
-                                const float* hp = ring + (long long)((sc - ctrl_delay) % H) * N * 3;
-                                ax = hp[0]; ay = hp[1]; az = hp[2];
-                            }
-                        }
-                        float* wp = ring + (long long)(sc % H) * N * 3;
-                        wp[0] = sx; wp[1] = sy; wp[2] = sz;
-                    }
+                    if (DR && P.dr_delay_hist > 0) delayed_command(P, env, N, s * 32 + lane, sc, ctrl_delay, ax, ay, az);
                     ax = clipf(ax, -1.0f, 1.0f); ay = clipf(ay, -1.0f, 1.0f); az = clipf(az, -1.0f, 1.0f);
                     nan_n += (ax == ax && ay == ay && az == az) ? 0u : 1u;   // (np.clip lets NaN through; counted)
-                    if (DR) {  // thrust noise: a <- a * (1 + sigma z), one normal per axis
+                    if (DR) {
                         const uint4 r = philox4x32_7(genv, ekey, (unsigned)sc, (unsigned)(s * 32 + lane) | (DR_STREAM_A << 16), P);
-                        ax = __fmul_rn(ax, __fmaf_rn(P.dr_std_thrust, dr_normal(P.dr_qtable, dr_field(r, 0)), 1.0f));
-                        ay = __fmul_rn(ay, __fmaf_rn(P.dr_std_thrust, dr_normal(P.dr_qtable, dr_field(r, 1)), 1.0f));
-                        az = __fmul_rn(az, __fmaf_rn(P.dr_std_thrust, dr_normal(P.dr_qtable, dr_field(r, 2)), 1.0f));
+                        thrust_noise(P, [=](int f) { return dr_normal(P.dr_qtable, dr_field(r, f)); }, ax, ay, az);
                     }
-                    v.x = __fadd_rn(v.x, __fmul_rn(__fmul_rn(ax, c_amax), c_dt));
-                    v.y = __fadd_rn(v.y, __fmul_rn(__fmul_rn(ay, c_amax), c_dt));
-                    v.z = __fadd_rn(v.z, __fmul_rn(__fmul_rn(az, c_amax), c_dt));
-                    const float speed = norm1d<0>(v.x, v.y, v.z);  // _clip_speed (:179-183)
-                    if (!(speed <= c_vmax || speed < P.eps_speed)) {
-                        v.x = __fmul_rn(__fdiv_rn(v.x, speed), c_vmax);
-                        v.y = __fmul_rn(__fdiv_rn(v.y, speed), c_vmax);
-                        v.z = __fmul_rn(__fdiv_rn(v.z, speed), c_vmax);
-                    }
-                    px[s] = __fadd_rn(px[s], __fmul_rn(v.x, c_dt));
-                    py[s] = __fadd_rn(py[s], __fmul_rn(v.y, c_dt));
-                    pz[s] = __fadd_rn(pz[s], __fmul_rn(v.z, c_dt));
+                    point_mass_step<0>(P, ax, ay, az, c_amax, c_vmax, c_dt, px[s], py[s], pz[s], v.x, v.y, v.z);
                 }
                 px[s] = clipf(px[s], -c_bound, c_bound);  // wall clip for ALL drones (:113-117)
                 py[s] = clipf(py[s], -c_bound, c_bound);
@@ -250,65 +221,25 @@ swarm_step_rotx_kernel(const DevParams P) {
         } else {
             // ================================ reset (:65-80) ================================
             __syncwarp();
-            const unsigned long long sh = P.rng[(long long)env * 4 + 0], sl = P.rng[(long long)env * 4 + 1];
-            const unsigned long long ih = P.rng[(long long)env * 4 + 2], il = P.rng[(long long)env * 4 + 3];
+            const Pcg64State rng = load_rng(P, env);
             double u_lo = P.rng_lo, u_range = P.rng_range;
             if (DR) {
-                // this episode's constants: 6 uniforms + an episode key from one counter per (env, reset)
-                const uint4 ra = philox4x32_10(genv, (unsigned)sl, (unsigned)(sl >> 32), DR_CTR_EPISODE, P);
-                const uint4 rb = philox4x32_10(genv, (unsigned)sl, (unsigned)(sl >> 32), DR_CTR_EPISODE + 1u, P);
-                const double inv24 = 1.0 / 16777216.0;
-                const double s_mass = __dadd_rn(P.dr_lo[0], __dmul_rn(P.dr_span[0], __dmul_rn((double)(ra.x >> 8), inv24)));
-                const double s_acc = __dadd_rn(P.dr_lo[1], __dmul_rn(P.dr_span[1], __dmul_rn((double)(ra.y >> 8), inv24)));
-                const double s_spd = __dadd_rn(P.dr_lo[2], __dmul_rn(P.dr_span[2], __dmul_rn((double)(ra.z >> 8), inv24)));
-                const double s_dt = __dadd_rn(P.dr_lo[3], __dmul_rn(P.dr_span[3], __dmul_rn((double)(ra.w >> 8), inv24)));
-                const double s_rad = __dadd_rn(P.dr_lo[4], __dmul_rn(P.dr_span[4], __dmul_rn((double)(rb.x >> 8), inv24)));
-                const double s_wld = __dadd_rn(P.dr_lo[5], __dmul_rn(P.dr_span[5], __dmul_rn((double)(rb.y >> 8), inv24)));
-                const double world = __dmul_rn(P.dr_world, s_wld);
-                const double half_w = __dmul_rn(world, 0.5);
-                u_lo = -half_w; u_range = __dsub_rn(half_w, -half_w);
+                const EpisodeDraw ep = draw_episode_constants(P, genv, rng.sl);
+                u_lo = ep.u_lo(); u_range = ep.u_range();
                 if (lane == 0) {
-                    float delay = 0.0f;  // this episode's control delay: 4th word of the second block
-                    if (P.dr_delay_count > 0) {
-                        const double uu = __dmul_rn((double)(rb.w >> 8), inv24);
-                        int pick = P.dr_delay_count - 1;
-#pragma unroll 1
-                        for (int k = P.dr_delay_count - 1; k >= 0; --k)
-                            if (uu < P.dr_delay_cum[k]) pick = k;
-                        delay = (float)P.dr_delay_values[pick];
-                    }
-                    P.dr_params[(long long)env * 2 + 0] =
-                        make_float4(__double2float_rn(__ddiv_rn(__dmul_rn(P.dr_max_accel, s_acc), s_mass)),
-                                    __double2float_rn(__dmul_rn(P.dr_max_speed, s_spd)),
-                                    __double2float_rn(__dmul_rn(P.dr_dt, s_dt)), __double2float_rn(half_w));
-                    P.dr_params[(long long)env * 2 + 1] =
-                        make_float4(__double2float_rn(__dadd_rn(P.dr_r_c, __dmul_rn(P.dr_r_o, s_rad))),
-                                    __uint_as_float(rb.z), __double2float_rn(world), delay);
+                    float4 d0, d1;
+                    episode_params(P, ep, d0, d1);
+                    P.dr_params[(long long)env * 2 + 0] = d0;
+                    P.dr_params[(long long)env * 2 + 1] = d1;
                 }
-                ekey = rb.z;  // (the dynamics constants are not needed to observe)
+                ekey = ep.key;  // (the dynamics constants are not needed to observe)
             }
-#pragma unroll 4
-            for (int k = lane; k < P.n_draws; k += 32) {
-                unsigned long long oh, ol;
-                pcg_jump(P.jump[k + 1], sh, sl, ih, il, oh, ol);
-                const float val = pcg_uniform_f32(oh, ol, u_lo, u_range);
-                if (k < 3 * N) {  // drone j = k / 3 lives at [slot j / 32][lane j % 32]
-                    const int j = k / 3;
-                    reinterpret_cast<float*>(tab2 + j)[k - 3 * j] = val;
-                } else if (k < 3 * N + 3) {
-                    reinterpret_cast<float*>(tgoal)[k - 3 * N] = val;
-                } else {
-                    const int kk = k - 3 * N - 3;
-                    reinterpret_cast<float*>(tobs + kk / 3)[kk % 3] = val;
-                }
-            }
+            // drone j lives at [slot j / 32][lane j % 32]
+            reset_env_draws<4>(
+                P, lane, N, rng, u_lo, u_range, [=](int j) { return reinterpret_cast<float*>(tab2 + j); },
+                [=]() { return reinterpret_cast<float*>(tgoal); }, [=](int m) { return reinterpret_cast<float*>(tobs + m); });
             if (lane == 0) {
-                unsigned long long oh, ol;
-                pcg_jump(P.jump[P.n_draws], sh, sl, ih, il, oh, ol);
-                P.rng[(long long)env * 4 + 0] = oh;
-                P.rng[(long long)env * 4 + 1] = ol;
-                P.step_count[env] = 0;
-                P.ep_return[env] = 0.0f;
+                reset_env_finish(P, env, rng);
                 reinterpret_cast<float*>(tgoal)[3] = 0.0f;
             }
             for (int k = lane; k < M; k += 32) reinterpret_cast<unsigned*>(tobs + k)[3] = (unsigned)k;
@@ -708,7 +639,6 @@ swarm_step_rotx_kernel(const DevParams P) {
             //  known after the last pass; its rows are written twice, as before.)
             if (STEP && P.auto_reset) doomed = doomed || __any_sync(FULL_MASK, (f & 2u) != 0u);
             if (!doomed) {
-                float* row = srow;
                 const float4 t0 = tab2[nj[0]], t1 = tab2[nj[1]];
                 const float4 t2 = tab2[nj[2]];
                 const float4 b0 = tobs[om[0]], b1 = tobs[om[1]], b2 = tobs[om[2]], b3 = tobs[om[3]];
@@ -716,19 +646,8 @@ swarm_step_rotx_kernel(const DevParams P) {
                 // block this step's thrust noise was cut from (a reset observation: step_count 0, counter 0xFFFFFFFF)
                 uint4 rA = make_uint4(0, 0, 0, 0);
                 if (DR) rA = philox4x32_7(genv, ekey, STEP ? (unsigned)sc : 0xFFFFFFFFu, (unsigned)me | (DR_STREAM_A << 16), P);
-                auto noisy = [&](float x, float sigma, int f) {
-                    return DR ? __fmaf_rn(sigma, dr_normal(P.dr_qtable, dr_field(rA, f)), x) : x;
-                };
-                row[0] = noisy(p_x, P.dr_std_pos, 3); row[1] = noisy(p_y, P.dr_std_pos, 4); row[2] = noisy(p_z, P.dr_std_pos, 5);
-                row[3] = noisy(vx[0], P.dr_std_vel, 6); row[4] = noisy(vy[0], P.dr_std_vel, 7); row[5] = noisy(vz[0], P.dr_std_vel, 8);
-                row[6] = __fsub_rn(gx, p_x); row[7] = __fsub_rn(gy, p_y); row[8] = __fsub_rn(gz, p_z);
-                row[9] = __fsub_rn(t0.x, p_x); row[10] = __fsub_rn(t0.y, p_y); row[11] = __fsub_rn(t0.z, p_z); row[12] = nd[0];
-                row[13] = __fsub_rn(t1.x, p_x); row[14] = __fsub_rn(t1.y, p_y); row[15] = __fsub_rn(t1.z, p_z); row[16] = nd[1];
-                row[17] = __fsub_rn(t2.x, p_x); row[18] = __fsub_rn(t2.y, p_y); row[19] = __fsub_rn(t2.z, p_z); row[20] = nd[2];
-                row[21] = __fsub_rn(b0.x, p_x); row[22] = __fsub_rn(b0.y, p_y); row[23] = __fsub_rn(b0.z, p_z); row[24] = noisy(od[0], P.dr_std_obst, 9);
-                row[25] = __fsub_rn(b1.x, p_x); row[26] = __fsub_rn(b1.y, p_y); row[27] = __fsub_rn(b1.z, p_z); row[28] = noisy(od[1], P.dr_std_obst, 10);
-                row[29] = __fsub_rn(b2.x, p_x); row[30] = __fsub_rn(b2.y, p_y); row[31] = __fsub_rn(b2.z, p_z); row[32] = noisy(od[2], P.dr_std_obst, 11);
-                row[33] = __fsub_rn(b3.x, p_x); row[34] = __fsub_rn(b3.y, p_y); row[35] = __fsub_rn(b3.z, p_z); row[36] = noisy(od[3], P.dr_std_obst, 12);
+                observe_row_k3s4<DR>(P, srow, p_x, p_y, p_z, vx[0], vy[0], vz[0], gx, gy, gz, t0, t1, t2, nd, b0, b1, b2, b3, od,
+                                     [=](int f) { return dr_normal(P.dr_qtable, dr_field(rA, f)); });
                 fence_async_smem();
                 __syncwarp();
                 if (lane == 0) {
